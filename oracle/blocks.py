@@ -32,10 +32,12 @@ def get_timestep_embedding(timesteps: torch.Tensor, embedding_dim: int, flip_sin
     half_dim = embedding_dim // 2
     exponent = -math.log(max_period) * torch.arange(0, half_dim, dtype=torch.float32, device=timesteps.device)
     exponent = exponent / (half_dim - downscale_freq_shift)
-    emb = torch.exp(exponent)
+    # fp32 exp / sin / cos are not correctly rounded and differ between CPU vector units: they are evaluated in fp64 and
+    # rounded once, so the fp32 embedding (and every golden vector downstream of it) is the same on every machine
+    emb = torch.exp(exponent.double()).float()
     emb = timesteps[:, None].float() * emb[None, :]
     emb = scale * emb
-    emb = torch.cat([torch.sin(emb), torch.cos(emb)], dim=-1)
+    emb = torch.cat([torch.sin(emb.double()), torch.cos(emb.double())], dim=-1).float()
     if flip_sin_to_cos:
         emb = torch.cat([emb[:, half_dim:], emb[:, :half_dim]], dim=-1)
     if embedding_dim % 2 == 1:
@@ -70,7 +72,9 @@ class TimestepEmbedding(nn.Module):
     def forward(self, sample, condition=None):
         if condition is not None:
             sample = sample + self.cond_proj(condition)
-        sample = self.linear_1(sample)
+        # get_timestep_embedding returns fp32 and the reference's adapter passes it on uncast: float64 parity runs
+        # need it in the layer's dtype (a no-op in fp32, and what autocast does anyway)
+        sample = self.linear_1(sample.to(self.linear_1.weight.dtype))
         sample = self.act(sample)
         sample = self.linear_2(sample)
         return sample

@@ -7,6 +7,17 @@ import torch
 
 from .weights import seeded_tensor
 
+
+def to_double(x):
+    """Floating-point tensors of a (nested) inputs structure in float64; everything else unchanged."""
+    if torch.is_tensor(x):
+        return x.double() if x.is_floating_point() else x
+    if isinstance(x, (list, tuple)):
+        return type(x)(to_double(v) for v in x)
+    if isinstance(x, dict):
+        return {k: to_double(v) for k, v in x.items()}
+    return x
+
 # residual shapes of the SD1.5 ControlNet for a base (latent) resolution r: 12 down tensors + mid
 CN_CHANNELS = [320, 320, 320, 320, 640, 640, 640, 1280, 1280, 1280, 1280, 1280]
 CN_DIV = [1, 1, 1, 2, 2, 2, 4, 4, 4, 8, 8, 8]

@@ -57,7 +57,7 @@ def sample_indices(numel: int, k: int = 512, seed: int = 1234) -> torch.Tensor:
 
 def fingerprint(t: torch.Tensor, k: int = 512) -> dict:
     """Compact, order-sensitive summary of a tensor used as a golden vector."""
-    f = t.detach().float().reshape(-1).cpu()
+    f = t.detach().double().reshape(-1).cpu()
     idx = sample_indices(f.numel(), k)
     return {
         "shape": list(t.shape),
